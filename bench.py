@@ -10,6 +10,7 @@ Weights are seeded synthetic checkpoints of the real architectures (no model fil
 N GPUs = N songs (one per rank, weak scaling, no data-path collective).
 
   python bench.py --gpus 1 --steps 3 --warmup 3              # our arm
+  python bench.py --gpus 1 --steps 3 --warmup 3 --dump-outputs DIR   # + the cover of the last timed step as DIR/*.npy
   python bench.py --impl reference --steps 1 --warmup 0      # CPU arm: the oracle restatement of the reference
   python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 Prints ONE JSON line on rank 0.
@@ -37,6 +38,7 @@ METRIC = "audio_seconds_per_second_full_cover_pipeline_4min_44k1_stereo"
 DTYPE_NOTE = ("fp16 operands (MDX-Net U-Net, tcgen05 kind::f16) + tf32 (other tensor-core GEMMs; rmvpe as 3xTF32 split operands), fp32 "
               "accumulate; fp32/fp64 row kernels")
 UNIT = "audio-s/s"
+DUMP_FRAMES = 1 << 21               # --dump-outputs: at most this many cover frames (16 MB float32 + 16 MB of row numbers)
 
 
 def synth_song(seconds: float, seed: int) -> np.ndarray:
@@ -183,6 +185,16 @@ def output_check(eng, song_dev, song_seconds):
                         "voiced_frac": round(float((pf_ref[:n] > 0).mean()), 3), "distinct_levels": int(len(np.unique(p_ref[:n]))),
                         "oracle_cpu_s": round(time.perf_counter() - t0, 1)}
     return res
+
+
+def dump_outputs(path, cover):
+    """The cover's int16 frames [n, 2] as float32 `path`/cover.npy and their row numbers as float64 `path`/cover_frames.npy:
+    all rows, or above DUMP_FRAMES a fixed seeded sample of them, so that two builds can be compared frame for frame."""
+    os.makedirs(path, exist_ok=True)
+    n = cover.shape[0]
+    rows = np.arange(n) if n <= DUMP_FRAMES else np.sort(np.random.default_rng(0).choice(n, DUMP_FRAMES, replace=False))
+    np.save(os.path.join(path, "cover.npy"), cover[rows].astype(np.float32))
+    np.save(os.path.join(path, "cover_frames.npy"), rows.astype(np.float64))
 
 
 def install_tc_profiler():
@@ -549,7 +561,13 @@ def main():
                     help="weak (default, BASELINE cfg 5): one song per GPU; strong (cfg 4 style): ONE song shared by all GPUs — MDX chunk "
                          "ranges per rank + all-gather, RVC segments round-robin after a broadcast F0")
     ap.add_argument("--no-output-check", action="store_true", help="skip the finite / non-silent / F0-parity check of the timed graph")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the cover returned by the last timed step to DIR (see dump_outputs); inputs and weights are seeded")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.config != "cover"):
+        ap.error("--dump-outputs writes the cover of the headline workload (--impl b200 --config cover)")
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
@@ -564,6 +582,7 @@ def main():
     if not torch.cuda.is_available():
         raise SystemExit("bench.py (b200 arm) needs a CUDA device; there is no CPU fallback")
     torch.cuda.set_device(local_rank)
+    torch.cuda.manual_seed(0)          # the synthesizer's noise draws: the same outputs from run to run
     device = f"cuda:{local_rank}"
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device(device))
@@ -628,6 +647,8 @@ def main():
 
     e2e_ms = timed_loop(e2e_step, args.steps)
     sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out_host["cover"])
     # ---- one more step OUTSIDE the timed regions with CUDA events around every tcgen05 tap-GEMM launch (the event
     # pairs perturb launch overlap, so they must not sit inside the step timing): per-kernel-family roofline data
     from aicovergen_b200 import plans

@@ -15,10 +15,27 @@ def sweep(seconds):
     return (0.5 * np.sin(2 * np.pi * (100 * t + 45 * t * t))).astype(np.float32)
 
 
+F0_RTOL = 1e-5
+
+
+def coarse_pitch_mismatches(f0, f0_ref):
+    """(frames whose coarse pitch index differs from the oracle's, frames that straddle a rounding boundary).  A frame
+    straddles when the two f0 values lie within F0_RTOL of each other on either side of a boundary of the quantiser: the
+    oracle then sits closer to the boundary than fp32 can place it (the trained-like weights hold the sweep near 776.4 Hz,
+    one such boundary, where one frame lies 4e-8 from it and the oracle alone moves by 1e-7 between CPU thread counts), so
+    either index is the reference's.  Every other frame must match exactly."""
+    from oracle import rmvpe as orm
+
+    pitch, pitch_ref = orm.coarse_pitch(f0, 0)[0], orm.coarse_pitch(f0_ref, 0)[0]
+    straddle = (np.abs(f0 - f0_ref) <= F0_RTOL * np.abs(f0_ref)) & (np.abs(pitch - pitch_ref) == 1)
+    return int(((pitch != pitch_ref) & ~straddle).sum()), int(straddle.sum())
+
+
 @pytest.mark.parametrize("weights", ["trained_like", "raw"])
 @pytest.mark.parametrize("seconds", [2.93, 10.0])
 def test_rmvpe_f0_parity(seconds, weights):
-    """BASELINE.json config 1 (10 s sweep) through the `infer_from_audio` plug point: coarse pitch indices bit-exact.
+    """BASELINE.json config 1 (10 s sweep) through the `infer_from_audio` plug point: f0 within F0_RTOL of the oracle and
+    coarse pitch indices bit-exact except across a rounding boundary (coarse_pitch_mismatches).
 
     Salience tolerance: a pure sine sweep leaves most mel bins at leakage level, right around the 1e-5 clamp of the
     log (rmvpe.py:324).  There the fp32 STFT's own rounding (~1e-6 absolute, whether FFT as in torch or DFT-GEMM as here)
@@ -45,15 +62,14 @@ def test_rmvpe_f0_parity(seconds, weights):
     print(f"[rmvpe {weights} {seconds}s] salience max abs err {err:.3e} over {tuple(sal.shape)}")
     f0 = net.infer_from_audio(x, thred=0.03)
     assert f0.shape == f0_ref.shape == (1 + len(x) // 160,)
-    pitch, pitchf = orm.coarse_pitch(f0, 0)
-    mism = int((pitch != pitch_ref).sum())
+    mism, straddle = coarse_pitch_mismatches(f0, f0_ref)
     both = (f0 > 0) & (f0_ref > 0)
     rel = np.abs(f0 - f0_ref)[both] / f0_ref[both]
-    print(f"[rmvpe {weights} {seconds}s] coarse-pitch mismatches {mism}/{len(pitch)}; f0 max rel diff {rel.max():.3e}; voiced "
-          f"{(f0_ref > 0).mean():.2f}; {len(np.unique(pitch_ref))} distinct levels")
+    print(f"[rmvpe {weights} {seconds}s] coarse-pitch mismatches {mism}/{len(f0)} (+{straddle} across a rounding boundary); "
+          f"f0 max rel diff {rel.max():.3e}; voiced {(f0_ref > 0).mean():.2f}; {len(np.unique(pitch_ref))} distinct levels")
     assert err < (1.5e-3 if weights == "trained_like" else 3e-4)
     assert mism == 0, "coarse pitch indices must match the reference bit for bit"
-    assert np.array_equal(f0 > 0, f0_ref > 0) and rel.max() < 1e-3
+    assert np.array_equal(f0 > 0, f0_ref > 0) and rel.max() < F0_RTOL
 
 
 @pytest.mark.parametrize("backend,bar", [(tg.BACKEND_TC, 5e-5), (tg.BACKEND_SIMT, 2e-5)])
